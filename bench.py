@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - images/sec of the FeMaSR x4 SR hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2|3|5|2test]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2|3|5|2test] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one encode_and_decode pass (`FeMaSRNet.forward`) over one batch of synthetic LR images:
@@ -19,6 +19,12 @@ test_tile(256,32) on one 1024x1024 image; 2test: config 2 through FeMaSRNet.test
             launching stream (engine profile mode, extra steps after the timed region)
   cpu_baseline  the CPU oracle port (the reference's ATen-CPU arithmetic) on this host's cores, bounded sample
 --impl reference runs only that CPU arm as the step and prints the same line shape.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (float32): `sr` (with N
+GPUs the all-gathered batch) and, for the forward entry, rank 0's `codebook_loss` and `indices`.  Inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output.  An array of more than
+DUMP_MAX_VALUES values is stored as the 1-D sample of its values at a fixed seeded set of sorted flat positions (the same
+set for every run of that shape), which keeps a dump under 64 MB.
 """
 from __future__ import annotations
 
@@ -44,6 +50,19 @@ CONFIGS = {
     "5": {"scale": 4, "lr": 1024, "batch": 1, "entry": "tile", "name": "config 5: test_tile(256, 32)"},
 }
 TILE, TILE_PAD = 256, 32
+DUMP_MAX_VALUES = 1 << 23       # 32 MB of float32 per dumped array
+
+
+def dump_array(path, t):
+    """Saves an output to `path` as float32 (float64 stays float64), sampled as described in the module docstring."""
+    import numpy as np
+    import torch
+    flat = t.detach().reshape(-1)
+    if flat.numel() > DUMP_MAX_VALUES:
+        pos = np.unique(np.random.default_rng(0).integers(0, flat.numel(), DUMP_MAX_VALUES))
+        t = flat[torch.from_numpy(pos).to(flat.device)]
+    a = t.detach().cpu().numpy()
+    np.save(path, a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def load_peaks():
@@ -193,7 +212,13 @@ def main():
     ap.add_argument("--e-dim", type=int, default=256)
     ap.add_argument("--gemm-path", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the CPU arm sizes its sample by timing, so its inputs vary)")
     cfgd = CONFIGS[args.config]
     args.batch = args.batch or cfgd["batch"]
     args.lr = args.lr or cfgd["lr"]
@@ -267,13 +292,15 @@ def main():
     eng = net._native(dev)
 
     def run_resident():
-        """One pass of the configuration's entry over the device-resident batch -> SR tensor."""
+        """One pass of the configuration's entry over the device-resident batch -> {name: tensor} as its caller receives
+        them (from a graph replay they live in the graph's static buffers until the next replay)."""
         if args.entry == "forward":
             # the engine's fixed launch list, replayed as a CUDA graph (same kernels, no per-launch host work)
-            return (eng.forward_graph(x_dev) if eng.use_graph else eng.forward(x_dev, want_indices=True, want_loss=True))[0]
+            y, loss, idx = eng.forward_graph(x_dev) if eng.use_graph else eng.forward(x_dev, want_indices=True, want_loss=True)
+            return {"sr": y, "codebook_loss": loss, "indices": idx}
         if args.entry == "test":
-            return eng.test(x_dev)
-        return eng.test_tile(x_dev, TILE, TILE_PAD)
+            return {"sr": eng.test(x_dev)}
+        return {"sr": eng.test_tile(x_dev, TILE, TILE_PAD)}
 
     def run_public(xd):
         """The same through the reference-facing surface (what a user of FeMaSRNet calls)."""
@@ -341,10 +368,10 @@ def main():
                                  "stream, overlapping the next step's forward; drained inside the timed region)")
 
     def step_resident():
-        out = run_resident()
+        outs = run_resident()
         if gather:
-            gather(out)
-        return out
+            gather(outs["sr"])
+        return outs
 
     def step_e2e():
         xd = x_host.to(dev, non_blocking=True)
@@ -360,11 +387,12 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms for `steps` calls of fn, what the last call returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         if gather:
             gather.drain()                      # the last step's all-gather belongs to the timed region
         e1.record()
@@ -373,15 +401,23 @@ def main():
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return ms.item()
+        return ms.item(), last
 
     for _ in range(args.warmup):
         step_resident()
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(step_resident, args.steps)
+    ms_total, last = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before anything else runs: the e2e pass below replays the same graph into the same static buffers
+        if gather:
+            last = dict(last, sr=gather.full[(gather.i - 1) & 1])      # every rank's shard of the last step
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in last.items():
+            dump_array(os.path.join(args.dump_outputs, f"{name}.npy"), t)
+        print(f"[bench] last timed step's outputs written to {args.dump_outputs}: {sorted(last)}", file=sys.stderr)
     # one eager pass with the engine's profile mode on: counts the kernels one step launches (and their FLOPs)
     eng.set_profile(True)
     if args.entry == "forward":
@@ -394,7 +430,7 @@ def main():
     flops_step = sum(v["flops"] for v in prof1.values())
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     # per-kernel CUDA-event timing (engine profile mode), 2 extra steps
     eng.set_profile(True)

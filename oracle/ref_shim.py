@@ -3,8 +3,7 @@
 The reference needs `timm` and `pyiqa`, neither installed here (network_swinir.py:11,
 losses/losses.py:11, models/femasr_model.py:15).  timm contributes no inference arithmetic
 (DropPath is nn.Identity at drop_path=0, network_swinir.py:204), so two stub modules are enough.
-Used only by tests/golden/make_golden.py and tests that are skipped when /root/reference is absent
-(it does not exist on the GPU box).
+Used only by tests/golden/make_golden.py: the tests compare with what it stored under tests/golden/.
 """
 from __future__ import annotations
 

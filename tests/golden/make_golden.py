@@ -7,10 +7,15 @@ Weights are not stored: they are re-created anywhere by femasr_b200.spec.random_
 (seeded per tensor name); a digest of the weights is stored so a drift in the generator is caught.
 Inputs are stored (small), together with the reference's outputs at the public boundary and a
 strided sample of its internal stage outputs (forward hooks on the reference modules).
+
+reference_boundary.json.gz records the reference's state_dict() inventory (name, shape, dtype) for every
+configuration of tests/test_boundary.py and the SHA-256 of its entry script, inference_femasr.py.
 """
 from __future__ import annotations
 
+import gzip
 import hashlib
+import json
 import os
 import sys
 
@@ -21,7 +26,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 
 from femasr_b200.spec import encode_depth, random_state_dict  # noqa: E402
-from oracle.ref_shim import import_reference  # noqa: E402
+from oracle.ref_shim import REFERENCE_ROOT, import_reference  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
@@ -72,10 +77,27 @@ def sample(t: torch.Tensor) -> np.ndarray:
     return t[:, ::17, ::3, ::3].contiguous().numpy()
 
 
+def write_reference_boundary(ref):
+    from tests.test_boundary import CONFIGS, IDS
+    inventory = {}
+    for (scale, cbs), cid in zip(CONFIGS, IDS):
+        net = ref.FeMaSRNet(codebook_params=cbs, LQ_stage=scale != 1, scale_factor=scale)
+        inventory[cid] = [[k, list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in net.state_dict().items()]
+    with open(os.path.join(REFERENCE_ROOT, "inference_femasr.py"), "rb") as f:
+        script_sha256 = hashlib.sha256(f.read()).hexdigest()
+    rec = {"state_dict": inventory, "inference_femasr.py": {"sha256": script_sha256}}
+    path = os.path.join(OUT, "reference_boundary.json.gz")
+    with open(path, "wb") as f:
+        f.write(gzip.compress(json.dumps(rec, sort_keys=True).encode(), mtime=0))
+    print(f"reference_boundary: {len(inventory)} state_dict inventories -> {os.path.getsize(path) / 1e3:.0f} kB")
+
+
 def main():
     ref = import_reference()
     torch.set_num_threads(max(1, os.cpu_count() or 1))
     only = set(sys.argv[1:])
+    if not only or "reference_boundary" in only:
+        write_reference_boundary(ref)
     for name, scale, e_dim, init, seed, entry, shape, extra in CASES + CPU_ONLY_CASES:
         if only and name not in only:
             continue

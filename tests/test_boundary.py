@@ -1,7 +1,10 @@
 """CPU: the parameter inventory (femasr_b200/spec.py), the drop-in module (basicsr/archs/femasr_arch.py) and the C
 engine's own spec agree with the REFERENCE's state_dict() - names, shapes, dtypes - for every supported configuration.
-The reference half runs only where /root/reference exists (the build container); the engine half runs everywhere."""
+The reference's inventories are stored in tests/golden/reference_boundary.json.gz (written by tests/golden/make_golden.py
+from the unmodified reference)."""
 import ctypes
+import gzip
+import json
 import os
 
 import pytest
@@ -15,26 +18,30 @@ CONFIGS = [
     (1, [[32, 1024, 256], [128, 256, 64]]),
 ]
 IDS = [f"x{s}_{len(c)}cb_e{c[0][2]}" for s, c in CONFIGS]
-HAVE_REF = os.path.isdir("/root/reference/basicsr")
+REFERENCE_BOUNDARY = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_boundary.json.gz")
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="the reference tree is only present in the build container")
+def reference_state_dict_inventory(cid):
+    """{name: (shape, dtype)} of the reference's FeMaSRNet(...).state_dict() for configuration `cid`."""
+    with gzip.open(REFERENCE_BOUNDARY, "rt") as f:
+        entries = json.load(f)["state_dict"][cid]
+    return {k: (tuple(shape), getattr(torch, dtype)) for k, shape, dtype in entries}
+
+
 @pytest.mark.parametrize("scale,cbs", CONFIGS, ids=IDS)
 def test_spec_matches_reference_state_dict(scale, cbs):
-    from oracle.ref_shim import import_reference
-    ref = import_reference()
-    net = ref.FeMaSRNet(codebook_params=cbs, LQ_stage=scale != 1, scale_factor=scale)
-    want = {k: (tuple(v.shape), v.dtype) for k, v in net.state_dict().items()}
+    want = reference_state_dict_inventory(IDS[CONFIGS.index((scale, cbs))])
     spec = {n: s for n, s, _k, _f in param_spec(scale, cbs[0][2], cbs[0][1], codebooks=cbs)}
     assert set(spec) == set(want), (sorted(set(spec) - set(want))[:5], sorted(set(want) - set(spec))[:5])
     for n, s in spec.items():
         assert tuple(s) == want[n][0], n
-    # a state_dict made here loads strictly into the reference, and the reference's loads strictly into ours
+    # a state_dict made here has the reference's keys and shapes (what its strict load checks), and one with the
+    # reference's keys, shapes and dtypes loads strictly into ours
     sd = random_state_dict(scale, cbs[0][2], seed=3, codebooks=cbs)
-    net.load_state_dict(sd, strict=True)
+    assert {k: tuple(v.shape) for k, v in sd.items()} == {k: s for k, (s, _d) in want.items()}
     from basicsr.archs.femasr_arch import FeMaSRNet
     mine = FeMaSRNet(codebook_params=cbs, LQ_stage=scale != 1, scale_factor=scale)
-    res = mine.load_state_dict(net.state_dict(), strict=True)
+    res = mine.load_state_dict({k: torch.zeros(s, dtype=d) for k, (s, d) in want.items()}, strict=True)
     assert not res.missing_keys and not res.unexpected_keys
     for k, v in mine.state_dict().items():
         assert v.dtype == want[k][1], k

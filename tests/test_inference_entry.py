@@ -1,5 +1,8 @@
 """Config 1 plumbing (image folder -> PNGs): the reference's own entry script against this repo's surface on
 CPU (must get as far as the device check), and the demo entry on the GPU against the oracle."""
+import gzip
+import hashlib
+import json
 import os
 import runpy
 import sys
@@ -12,9 +15,10 @@ import torch
 from basicsr.utils import img2tensor, tensor2img
 from femasr_b200.spec import random_state_dict
 from oracle import femasr_oracle as O
-from oracle.ref_shim import REFERENCE_ROOT, reference_available
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# the reference's entry script, committed verbatim as a test input (tests/fixtures/README.md)
+ENTRY_SCRIPT = os.path.join(ROOT, "tests", "fixtures", "inference_femasr.py")
 
 
 def _write_inputs(folder, sizes, seed=3):
@@ -39,7 +43,7 @@ def test_image_helpers_roundtrip():
     assert tensor2img(torch.full((1, 3, 2, 2), 1.7)).max() == 255     # clamp before scaling
 
 
-@pytest.mark.skipif(not reference_available() or torch.cuda.is_available(), reason="needs /root/reference and no GPU")
+@pytest.mark.skipif(torch.cuda.is_available(), reason="checks the behaviour without a GPU")
 def test_reference_entry_script_runs_unchanged_up_to_the_device(tmp_path, built_lib):
     """inference_femasr.py of the reference, unmodified, imports our basicsr, builds and loads the network and
     reads the image; without a GPU it must stop exactly at the first compute call (no CPU fallback)."""
@@ -51,18 +55,18 @@ def test_reference_entry_script_runs_unchanged_up_to_the_device(tmp_path, built_
     sys.argv = ["inference_femasr.py", "-s", "4", "-i", ins[0], "-o", str(tmp_path / "out"), "-w", str(w)]
     try:
         with pytest.raises(FemasrError, match="CUDA sm_100"):
-            runpy.run_path(os.path.join(REFERENCE_ROOT, "inference_femasr.py"), run_name="__main__")
+            runpy.run_path(ENTRY_SCRIPT, run_name="__main__")
     finally:
         sys.argv = argv
 
 
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference")
 def test_fixture_is_the_reference_script():
-    """tests/fixtures/inference_femasr.py (what the GPU box executes, tests/test_reference_entry_gpu.py) must be the
-    reference's entry script byte for byte."""
-    a = open(os.path.join(ROOT, "tests", "fixtures", "inference_femasr.py"), "rb").read()
-    b = open(os.path.join(REFERENCE_ROOT, "inference_femasr.py"), "rb").read()
-    assert a == b
+    """tests/fixtures/inference_femasr.py (what tests/test_reference_entry_gpu.py executes) must be the reference's
+    entry script byte for byte: its SHA-256 is the one tests/golden/make_golden.py recorded from the reference."""
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "reference_boundary.json.gz"), "rt") as f:
+        want = json.load(f)["inference_femasr.py"]["sha256"]
+    with open(ENTRY_SCRIPT, "rb") as f:
+        assert hashlib.sha256(f.read()).hexdigest() == want
 
 
 @pytest.mark.gpu
