@@ -48,31 +48,6 @@ def _digest(paths) -> str:
     return h.hexdigest()
 
 
-def build_variant(out_name: str, defines, verbose: bool = False) -> str:
-    """Experimental variant of the library (extra -D flags) next to the default one; selected with FEMASR_LIB."""
-    nvcc = _nvcc()
-    odir = os.path.join(OBJ, out_name)
-    os.makedirs(odir, exist_ok=True)
-    objs = []
-    for src in sources():
-        obj = os.path.join(odir, os.path.basename(src)[:-3] + ".o")
-        cmd = [nvcc, *NVCC_FLAGS, *[f"-D{d}" for d in defines], "-c", src, "-o", obj]
-        if verbose:
-            cmd.insert(1, "-Xptxas=-v")
-        r = subprocess.run(cmd, capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError(f"nvcc failed for {src}:\n{r.stdout}\n{r.stderr}")
-        if verbose:
-            print(r.stderr)
-        objs.append(obj)
-    out = os.path.join(HERE, out_name)
-    r = subprocess.run([nvcc, "-shared", "-o", out, *objs, "-gencode", "arch=compute_100a,code=sm_100a", "-lcudart"],
-                       capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    return out
-
-
 def build(force: bool = False, verbose: bool = False) -> str:
     srcs = sources()
     deps = srcs + [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]

@@ -123,10 +123,7 @@ constexpr int KV_LD = 40;   // row stride in halves (80 B): the 8 row addresses 
 
 // 7 resident CTAs per SM (72 registers): measured 0.139 ms per layer vs 0.141 at 6 (80 registers) and 0.181 when the
 // compiler is left free to use more registers
-#ifndef FEMASR_ATTN_MINBLOCKS
-#define FEMASR_ATTN_MINBLOCKS 7
-#endif
-__global__ void __launch_bounds__(128, FEMASR_ATTN_MINBLOCKS) window_attention_mma_kernel(const float* __restrict__ qkv,
+__global__ void __launch_bounds__(128, 7) window_attention_mma_kernel(const float* __restrict__ qkv,
                                                                    const float* __restrict__ bias_frag,
                                                                    float* __restrict__ out, __half* __restrict__ out_hi,
                                                                    __half* __restrict__ out_lo, int H, int W, int C,

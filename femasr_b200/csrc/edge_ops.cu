@@ -11,11 +11,9 @@ namespace femasr {
 // in_conv: 4x4, pad 1, Cin = 3.  Thread = (4 output channels) x (4 consecutive output pixels of one row): the
 // 4x7x3 input patch lives in registers (loads are shared by all channel-quad threads of the pixel group through
 // L1), every weight float4 is used for 16 FMAs, and the 4 stores per thread are contiguous across the warp's
-// channel quads.  SPLIT: write the fp16 hi/lo operand planes of the following tensor-core conv instead of fp32.
-template <bool SPLIT>
+// channel quads.
 __global__ void __launch_bounds__(256) in_conv_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                       const float* __restrict__ bias, float* __restrict__ y,
-                                                      __half* __restrict__ yhi, __half* __restrict__ ylo,
                                                       int B, int H, int W, int Cout) {
   constexpr int KS = 4, CIN = 3, PX = 4;
   const int Ho = H - 1, Wo = W - 1;
@@ -65,20 +63,7 @@ __global__ void __launch_bounds__(256) in_conv_kernel(const float* __restrict__ 
     const int ox = ox0 + p;
     if (ox >= Wo) break;
     const long e = ((((long)b * Ho + oy) * Wo + ox) * Cout) + q * 4;
-    if (SPLIT) {
-      const float v[4] = {acc[p].x, acc[p].y, acc[p].z, acc[p].w};
-      __align__(8) __half h[4], l[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const float cl = fminf(fmaxf(v[k], -65504.f), 65504.f);
-        h[k] = __float2half_rn(cl);
-        l[k] = __float2half_rn(cl - __half2float(h[k]));
-      }
-      *reinterpret_cast<uint2*>(yhi + e) = *reinterpret_cast<const uint2*>(h);
-      *reinterpret_cast<uint2*>(ylo + e) = *reinterpret_cast<const uint2*>(l);
-    } else {
-      *reinterpret_cast<float4*>(y + e) = acc[p];
-    }
+    *reinterpret_cast<float4*>(y + e) = acc[p];
   }
 }
 
@@ -212,32 +197,16 @@ __global__ void copy_window_kernel(const float* __restrict__ src, float* __restr
 
 using namespace femasr;
 
-static int in_conv_launch(const float* x, const float* w, const float* bias, float* y, void* yhi, void* ylo, int B,
-                          int Cin, int H, int W, int Cout, void* stream) {
-  FEMASR_CHECK_ARG(x && w && (y || (yhi && ylo)), "in_conv: null pointer");
+extern "C" int femasr_in_conv4x4(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int H,
+                                 int W, int Cout, void* stream) {
+  FEMASR_CHECK_ARG(x && w && y, "in_conv: null pointer");
   FEMASR_CHECK_ARG(B > 0 && H >= 3 && W >= 3 && Cin == 3, "in_conv: needs Cin == 3 and H, W >= 3");
   FEMASR_CHECK_ARG(Cout % 4 == 0 && 256 % (Cout / 4) == 0 && Cout <= 1024, "in_conv: unsupported Cout");
   const long ngrp = (long)B * (H - 1) * cdiv(W - 1, 4);
   const int gpb = 256 / (Cout / 4);
   const unsigned grid = (unsigned)cdiv(ngrp, gpb);
-  if (y)
-    in_conv_kernel<false><<<grid, 256, 0, as_stream(stream)>>>(x, w, bias, y, nullptr, nullptr, B, H, W, Cout);
-  else
-    in_conv_kernel<true><<<grid, 256, 0, as_stream(stream)>>>(x, w, bias, nullptr, reinterpret_cast<__half*>(yhi),
-                                                                reinterpret_cast<__half*>(ylo), B, H, W, Cout);
+  in_conv_kernel<<<grid, 256, 0, as_stream(stream)>>>(x, w, bias, y, B, H, W, Cout);
   return launch_status("in_conv_kernel");
-}
-
-extern "C" int femasr_in_conv4x4(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int H,
-                                 int W, int Cout, void* stream) {
-  FEMASR_CHECK_ARG(y, "in_conv: null output");
-  return in_conv_launch(x, w, bias, y, nullptr, nullptr, B, Cin, H, W, Cout, stream);
-}
-
-extern "C" int femasr_in_conv4x4_split(const float* x, const float* w, const float* bias, void* y_hi, void* y_lo, int B,
-                                       int Cin, int H, int W, int Cout, void* stream) {
-  FEMASR_CHECK_ARG(y_hi && y_lo, "in_conv_split: null output");
-  return in_conv_launch(x, w, bias, nullptr, y_hi, y_lo, B, Cin, H, W, Cout, stream);
 }
 
 // in_conv on the tensor cores: the 4x4x3 patch of every output pixel as one K = 48 (padded to 64) row of split-fp16

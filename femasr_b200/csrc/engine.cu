@@ -108,13 +108,7 @@ struct femasr_net {
   std::map<std::string, Tap> taps;
   int last_launches = 0;
   bool profile = false;
-  bool tc_precise = true;                 // K-sliced fp32 accumulation for the layers in front of the VQ
-  bool oc_mma = true;                     // out_conv on mma.sync in the tensor-core path (FEMASR_OUTCONV_MMA=0: SIMT kernel)
   bool f8_cross = true;                   // layers behind the VQ: the two cross products of the split as one fp8 product (FEMASR_F8_CROSS=0: three fp16 products)
-  bool in_conv_tc = true;                 // in_conv as an im2col GEMM on the tensor cores (FEMASR_IN_CONV_TC=0: fp32 SIMT kernel)
-  int tc_slice_kb = 4;                    // K-slice length in 64-wide k-blocks (FEMASR_TC_SLICE_KB; study knob)
-  bool vq_fused = true;                   // VQ distances on the tensor cores with the argmin fused (FEMASR_VQ_FUSED=0: fp32 SIMT z.E^T + vq_select)
-  bool fast_silu = true;                  // approximate-unit SiLU in the operand staging behind the VQ (FEMASR_FAST_SILU=0: exact)
   std::vector<ProfRec> prof;
   std::string prof_json;
   ~femasr_net() {
@@ -131,6 +125,10 @@ struct femasr_net {
 };
 
 namespace femasr {
+
+// K-sliced accumulation of the tensor-core convs in front of the VQ: the truncating MMA accumulator is folded into an
+// fp32 running sum every TC_SLICE_KB 64-wide k-blocks (256 of K)
+constexpr int TC_SLICE_KB = 4;
 
 static int chan(int res) {
   switch (res) { case 8: case 16: case 32: case 64: return 256; case 128: return 128; case 256: return 64; case 512: return 32; }
@@ -315,7 +313,7 @@ struct Ctx {
       const bool f8 = relaxed && net->f8_cross && !pre_hi && ksize == 3 && prologue != FEMASR_PRO_LN &&
                       (upsample ? net->tcw_up8.count(wname + ".weight") : net->tcw8.count(wname + ".weight")) != 0;
       if (!pre_hi) {
-        const int pmode = (prologue == FEMASR_PRO_GN_SILU && relaxed && net->fast_silu) ? FEMASR_PRO_GN_SILU_FAST : prologue;
+        const int pmode = (prologue == FEMASR_PRO_GN_SILU && relaxed) ? FEMASR_PRO_GN_SILU_FAST : prologue;
         run(detail_name(f8 ? "tc_prepare_f8" : "tc_prepare", pmode, Cin, Cin, Hin, Win, 0, 1, 0), 0.0, [&] {
           return f8 ? femasr_tc_prepare_f8(x, ahi, alo, pmode, pa, pb, B, Hin, Win, Cin, st)
                     : femasr_tc_prepare(x, ahi, alo, pmode, pa, pb, gamma, beta, B, Hin, Win, Cin, 0,
@@ -336,11 +334,10 @@ struct Ctx {
       const int Ho = stride == 2 ? (Hin - 1) / 2 + 1 : Hin * u, Wo = stride == 2 ? (Win - 1) / 2 + 1 : Win * u;
       const double flops = 2.0 * B * Ho * (double)Wo * Cout * Cin * ksize * ksize;   // algorithmic (reference) count
       const int nkb = (upsample ? 4 : ksize * ksize) * (Cin / 64);
-      const int slice = net->tc_slice_kb;        // k-blocks per accumulator drain (default 4 = 256 of K)
-      if ((precise || precise_region) && net->tc_precise && nkb > slice) {
+      if ((precise || precise_region) && nkb > TC_SLICE_KB) {
         // K-sliced accumulation (layers in front of the VQ): every 256 of K the tensor core's truncating accumulator
         // is folded into an fp32 round-to-nearest running sum held in TMEM (see femasr_tc_args.slice_kb)
-        t.slice_kb = slice;
+        t.slice_kb = TC_SLICE_KB;
       }
       run(detail_name("tc_igemm", ksize, Cin, Cout, Hin, Win, upsample, stride, t.slice_kb), flops,
           [&] { return femasr_tc_igemm(&t, st); });
@@ -364,7 +361,7 @@ struct Ctx {
     memset(&t, 0, sizeof(t));
     t.B = B; t.H = H; t.W = W; t.Cin = Cin; t.Cout = Cout; t.ksize = 3; t.upsample = upsample; t.stride = stride;
     t.pair = -1; t.strip = -1;
-    t.slice_kb = (precise_region && net->tc_precise && (upsample ? 4 : 9) * (Cin / 64) > net->tc_slice_kb) ? net->tc_slice_kb : 0;
+    t.slice_kb = (precise_region && (upsample ? 4 : 9) * (Cin / 64) > TC_SLICE_KB) ? TC_SLICE_KB : 0;
     Stats st_;
     st_.rows = femasr_tc_gn_partial_rows(&t);
     st_.partial = ar.alloc((size_t)B * st_.rows * 32 * 2);
@@ -497,7 +494,7 @@ struct Ctx {
     conv("before_quant_group." + ks, src, z, B, hh, ww, Cin, e, 1, 1, 0, FEMASR_PRO_NONE, nullptr, nullptr, nullptr, nullptr, 0, nullptr, nullptr);
     tap(k == 0 ? "z" : (k == 1 ? "z1" : "z2"), z, N * e);
     const std::string cname = "quantize_group." + ks + ".embedding.weight";
-    const bool fused = net->cfg.gemm_path == 1 && net->vq_fused && (dry() || net->tcw.count(cname) != 0);
+    const bool fused = net->cfg.gemm_path == 1 && (dry() || net->tcw.count(cname) != 0);
     // fused: tensor-core distances + in-kernel top-4 (no [N, n_e] tensor); else the fp32 SIMT product + vq_select
     float *zc = nullptr, *arow = nullptr, *zhi = nullptr, *zlo = nullptr, *cand = nullptr;
     if (fused) {
@@ -620,8 +617,8 @@ struct Ctx {
       const float *ow = P("out_conv.weight"), *ob = P("out_conv.bias");
       const float* d2 = t;
       run("out_conv", 2.0 * 9 * 64 * 3 * (double)B * 64 * h * w,
-          [&] { return net->cfg.gemm_path == 1 && net->oc_mma ? femasr_out_conv3x3_mma(d2, ow, ob, y_nchw, B, 8 * h, 8 * w, 64, st)
-                                                               : femasr_out_conv3x3(d2, ow, ob, y_nchw, B, 8 * h, 8 * w, 64, st); });
+          [&] { return net->cfg.gemm_path == 1 ? femasr_out_conv3x3_mma(d2, ow, ob, y_nchw, B, 8 * h, 8 * w, 64, st)
+                                               : femasr_out_conv3x3(d2, ow, ob, y_nchw, B, 8 * h, 8 * w, 64, st); });
     }
     ar.release(t);
   }
@@ -643,33 +640,32 @@ struct Ctx {
     if (!tc || want_in_tap) {     // identical in the dry (sizing) run and the real run: taps are registered first
       cur = ar.alloc(in_elems);
       const int c0 = c;
-      if (!tc || want_in_tap)
-        run("in_conv", in_flops, [&] { return femasr_in_conv4x4(x_nchw, iw, ib, cur, B, cfg.in_channel, H, W, c0, st); });
+      run("in_conv", in_flops, [&] { return femasr_in_conv4x4(x_nchw, iw, ib, cur, B, cfg.in_channel, H, W, c0, st); });
       tap("in_conv", cur, in_elems);
     }
     if (tc) {
+      // K = 48 (-> 64) GEMM over im2col rows on the tensor cores, writing the down conv's split planes; set_param packs
+      // its weight blob (#im2col) for every in_conv of the tensor-core path
       in_hi = ar.alloc((in_elems + 1) / 2);
       in_lo = ar.alloc((in_elems + 1) / 2);
-      const int c0 = c;
-      const std::string wkey = enc + ".in_conv.weight#im2col";
-      if (net->in_conv_tc && (dry() || net->tcw.count(wkey))) {
-        // K = 48 (-> 64) GEMM over im2col rows on the tensor cores, writing the down conv's split planes
-        const size_t rows = (size_t)B * h * w;
-        float* ic_hi = ar.alloc(rows * 64 / 2);
-        float* ic_lo = ar.alloc(rows * 64 / 2);
+      const size_t rows = (size_t)B * h * w;
+      float* ic_hi = ar.alloc(rows * 64 / 2);
+      float* ic_lo = ar.alloc(rows * 64 / 2);
+      if (!dry() && ok()) {
+        const std::string wkey = enc + ".in_conv.weight#im2col";
+        const auto wt = net->tcw.find(wkey);
+        if (wt == net->tcw.end() || !wt->second.p) check(fail(FEMASR_ERR_STATE, "tensor-core weight not packed: " + wkey));
         run("in_conv_im2col", 0.0, [&] { return femasr_in_conv_im2col(x_nchw, ic_hi, ic_lo, B, cfg.in_channel, H, W, st); });
-        if (!dry() && ok()) {
+        if (ok()) {
           femasr_tc_args t;
           memset(&t, 0, sizeof(t));
-          t.a_hi = ic_hi; t.a_lo = ic_lo; t.w_blob = net->tcw[wkey].p; t.bias = ib;
+          t.a_hi = ic_hi; t.a_lo = ic_lo; t.w_blob = wt->second.p; t.bias = ib;
           t.out_hi = in_hi; t.out_lo = in_lo;
-          t.B = B; t.H = h; t.W = w; t.Cin = 64; t.Cout = c0; t.ksize = 1; t.stride = 1; t.pair = -1; t.strip = -1;
+          t.B = B; t.H = h; t.W = w; t.Cin = 64; t.Cout = c; t.ksize = 1; t.stride = 1; t.pair = -1; t.strip = -1;
           run("in_conv", in_flops, [&] { return femasr_tc_igemm(&t, st); });
         }
-        ar.release(ic_lo); ar.release(ic_hi);
-      } else {
-        run("in_conv", in_flops, [&] { return femasr_in_conv4x4_split(x_nchw, iw, ib, in_hi, in_lo, B, cfg.in_channel, H, W, c0, st); });
       }
+      ar.release(ic_lo); ar.release(ic_hi);
     }
     // which enc_feats the decoder loop reads: at quantising levels (before_quant input) and, in the LQ stage with
     // use_residual, at the other levels > 0 (skip adds)
@@ -749,7 +745,7 @@ static int check_geometry(femasr_net* net, int B, int H, int W) {
 }  // namespace femasr
 
 extern "C" const char* femasr_last_error(void) { return g_err.c_str(); }
-extern "C" int femasr_abi_version(void) { return 4; }   // 3: fused VQ + im2col in_conv entries; 4: femasr_tc_args.f8 + the F8 staging / packing entries
+extern "C" int femasr_abi_version(void) { return 5; }   // 3: fused VQ + im2col in_conv entries; 4: femasr_tc_args.f8 + the F8 staging / packing entries; 5: femasr_in_conv4x4_split removed
 
 extern "C" int femasr_device_cc(void) {
   int dev = 0;
@@ -789,13 +785,7 @@ extern "C" int femasr_net_create(const femasr_net_config* cfg, femasr_net** out)
   }
   n->depth = cfg->scale_factor == 4 ? 1 : (cfg->scale_factor == 2 ? 2 : 3);
   n->hq = cfg->scale_factor == 1;
-  if (const char* ev = getenv("FEMASR_TC_PRECISE")) n->tc_precise = atoi(ev) != 0;
-  if (const char* ev = getenv("FEMASR_FAST_SILU")) n->fast_silu = atoi(ev) != 0;
-  if (const char* ev = getenv("FEMASR_OUTCONV_MMA")) n->oc_mma = atoi(ev) != 0;
-  if (const char* ev = getenv("FEMASR_VQ_FUSED")) n->vq_fused = atoi(ev) != 0;
-  if (const char* ev = getenv("FEMASR_IN_CONV_TC")) n->in_conv_tc = atoi(ev) != 0;
   if (const char* ev = getenv("FEMASR_F8_CROSS")) n->f8_cross = atoi(ev) != 0;
-  if (const char* ev = getenv("FEMASR_TC_SLICE_KB")) n->tc_slice_kb = std::max(1, atoi(ev));
   build_spec(n);
   *out = n;
   return FEMASR_OK;
@@ -821,7 +811,7 @@ extern "C" int femasr_net_set_param(femasr_net* net, const char* name, const flo
     if (!pb.p) { FEMASR_CUDA(cudaMalloc(&pb.p, numel * sizeof(float))); pb.n = numel; }
     int s = femasr_pack_weight(rb.p, pb.p, pi.Cout, pi.Cin, pi.k, pi.k, st);
     if (s) return s;
-    if (net->cfg.gemm_path == 1 && net->in_conv_tc && pi.k == 4 && pi.Cin == 3 && pi.Cout % 64 == 0) {
+    if (net->cfg.gemm_path == 1 && pi.k == 4 && pi.Cin == 3 && pi.Cout % 64 == 0) {
       // in_conv as a K = 48 -> 64 tensor-core GEMM over im2col rows: [Cout][64] padded matrix -> split-fp16 blob
       float* tmp = nullptr;
       FEMASR_CUDA(cudaMallocAsync(&tmp, (size_t)pi.Cout * 64 * sizeof(float), st));
@@ -882,7 +872,7 @@ extern "C" int femasr_net_set_param(femasr_net* net, const char* name, const flo
     if (!eb.p) { FEMASR_CUDA(cudaMalloc(&eb.p, pi.Cout * sizeof(float))); eb.n = pi.Cout; }
     s = femasr_row_sumsq(rb.p, eb.p, pi.Cout, pi.Cin, st);
     if (s) return s;
-    if (net->cfg.gemm_path == 1 && net->vq_fused) {     // split-fp16 planes of the [n_e, e_dim] embedding: B operand of the fused VQ
+    if (net->cfg.gemm_path == 1) {     // split-fp16 planes of the [n_e, e_dim] embedding: B operand of the fused VQ
       DevBuf& tb = net->tcw[key];
       const size_t bytes = femasr_tc_weight_bytes(pi.Cout, pi.Cin, 1, 1);
       if (!tb.p) { FEMASR_CUDA(cudaMalloc(&tb.p, bytes)); tb.n = bytes / sizeof(float); }

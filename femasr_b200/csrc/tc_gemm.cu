@@ -68,14 +68,12 @@ __device__ __forceinline__ uint64_t global_ns() {
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-#ifndef FEMASR_MBAR_HINT_NS
-#define FEMASR_MBAR_HINT_NS 20000u
-#endif
+constexpr uint32_t MBAR_HINT_NS = 20000u;
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return;
   const uint64_t t0 = global_ns();
   uint32_t spins = 0;
-  while (!(FEMASR_MBAR_HINT_NS ? mbar_try_wait_hint(bar, parity, FEMASR_MBAR_HINT_NS) : mbar_try_wait(bar, parity))) {
+  while (!mbar_try_wait_hint(bar, parity, MBAR_HINT_NS)) {
     if ((++spins & 0xFFFu) == 0 && global_ns() - t0 > 4000000000ull) {   // 4 s: far beyond any legitimate wait
       printf("femasr tc_gemm: mbarrier wait timed out (block %d thread %d bar %u parity %u)\n", blockIdx.x, threadIdx.x, bar, parity);
       __trap();
@@ -109,13 +107,6 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }   // sources reusable
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }          // writes complete
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// Programmatic dependent launch: a kernel launched with the programmatic-serialisation attribute may start (its CTAs
-// become resident as the predecessor's retire, it runs its prologue) before the predecessor has finished;
-// griddepcontrol.wait blocks until the predecessor grid has completed and its memory is visible.  Both are no-ops in a
-// plain launch.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // One lane of a converged warp (elect.sync).  The single-thread roles (TMA producer, MMA issuer) are entered through this
 // instead of `lane == 0`: with a data-dependent lane test ptxas must assume several lanes with different operands may be
@@ -247,10 +238,7 @@ constexpr int TC_BM = 128, TC_BK = 64;
 // epilogue warps per TMEM lane quarter (= column split of the accumulator): 4 (16 epilogue warps) for the 128/256-wide
 // tiles - measured +4 % end to end over 8 warps, the short-K layers are epilogue-issue bound - but 2 for the 64-wide
 // tiles, where a warp would own a single 16-column chunk and the per-tile fixed work dominates (measured -15 %).
-#ifndef FEMASR_NSPLIT_WIDE
-#define FEMASR_NSPLIT_WIDE 4      // study knob: 2 = 8 epilogue warps with 168 registers each for the 128 / 256-wide tiles
-#endif
-constexpr int nsplit_for(int BN) { return BN == 64 ? 2 : FEMASR_NSPLIT_WIDE; }
+constexpr int nsplit_for(int BN) { return BN == 64 ? 2 : 4; }
 constexpr int tc_threads_for(int BN) { return 128 + 32 * 4 * nsplit_for(BN); }
 constexpr int A_PLANE_BYTES = TC_BM * TC_BK * 2;   // 16 KB
 
@@ -263,10 +251,6 @@ constexpr int A_PLANE_BYTES = TC_BM * TC_BK * 2;   // 16 KB
 // (the swizzle follows absolute address bits, see the MMA issuer).  Activation traffic from L2 drops 2.9x (3 loads
 // instead of 9 per chunk) - the narrow layers are L2->SM bound (profiles/tc_igemm_traffic_r1.json).  Weights stream
 // through their own ring, one tap per stage.
-#ifndef FEMASR_BRES_MERGE
-#define FEMASR_BRES_MERGE 1       // 0: one N = 64 MMA per (output row, tap) in the resident-weight strip kernel (A/B knob)
-#endif
-constexpr bool BRES_MERGE = FEMASR_BRES_MERGE != 0;
 constexpr int STRIP_PX = 130;                         // 128 outputs + one halo pixel each side
 constexpr int STRIP_PLANE_BYTES = 17 * 1024;          // 130 rows x 128 B = 16,640 B, padded to the 1024-B swizzle period
 
@@ -421,7 +405,6 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
   };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();        // the next kernel of the stream may begin its own prologue as our CTAs retire
   if (threadIdx.x == 0) {
     for (int s = 0; s < Cfg::NBAR_PIPE; ++s) mbar_init(bar_base + 8u * s, 1);
     // tmem-empty: ONE arrival per epilogue warp (of both CTAs when paired), by an elected lane after __syncwarp - 512
@@ -444,7 +427,6 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
   tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
-  pdl_wait();                     // barriers initialised, TMEM allocated: from here on the predecessor's output is read
 
   const int ksz = p.taps == 9 ? 3 : 1;   // (p.up: taps == 4, offsets from the phase)
 
@@ -476,13 +458,13 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
     if (BRES) {
       // the whole [64][9*64] weight matrix (hi, lo) once.  Merged layout (see the MMA issuer): per kw the hi planes of
       // kh = 2, 1, 0 back to back (3 x 8 KB), then the three lo planes - any run of consecutive kh is ONE B operand of
-      // N = 64, 128 or 192 rows.  Plain layout: tap t at smem_base + t * 2 * B_PLANE_BYTES.
+      // N = 64, 128 or 192 rows.
       const uint32_t bres_bar = bar_base + 8u * (2 * Cfg::SA_STAGES);
       mbar_expect_tx(bres_bar, Cfg::B_RES_BYTES);
       for (int tap = 0; tap < 9; ++tap) {
         const int kh = tap / 3, kw = tap - 3 * kh;
-        const uint32_t dst_hi = BRES_MERGE ? smem_base + (kw * 6 + (2 - kh)) * Cfg::B_PLANE_BYTES : smem_base + tap * 2 * Cfg::B_PLANE_BYTES;
-        const uint32_t dst_lo = dst_hi + (BRES_MERGE ? 3 : 1) * Cfg::B_PLANE_BYTES;
+        const uint32_t dst_hi = smem_base + (kw * 6 + (2 - kh)) * Cfg::B_PLANE_BYTES;
+        const uint32_t dst_lo = dst_hi + 3 * Cfg::B_PLANE_BYTES;
         tma_load_2d(dst_hi, &map_b_hi, bres_bar, tap * p.Cin, 0);
         tma_load_2d(dst_lo, &map_b_lo, bres_bar, tap * p.Cin, 0);
       }
@@ -548,7 +530,7 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
     int set = 0; uint32_t set_phase = 0;           // accumulator set (MR slots) of the current work item
     if (BRES) { mbar_wait(bar_base + 8u * (2 * Cfg::SA_STAGES), 0u); tc_fence_after(); }   // weights resident
     for (int work = worker; work < num_work; work += nworkers) {
-      if constexpr (BRES && BRES_MERGE) {
+      if constexpr (BRES) {
         // Multi-row strip tiles with MERGED tap rows.  ncu on these convs (profiles/ncu_r2_epilogue.json): the tensor-core
         // pipe 81 % utilised with its math sub-pipe at 42 % - a 128 x 64 x 16 MMA streams 4 KB of A and 2 KB of B out of
         // shared memory (~48 cycles at 128 B / clk) for 34 cycles of fp16 math (17 of e4m3 math): with N = 64 the operand
@@ -606,7 +588,7 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
           if (++sa == Cfg::SA_STAGES) { sa = 0; pa ^= 1u; }
         }
       } else
-      for (int sr = 0; sr < MR + 2; ++sr)
+      for (int sr = 0; sr < MR + 2; ++sr)                // streamed weights: one tap's weight tile per ring stage
         for (int cc = 0; cc < p.cchunks; ++cc) {
           mbar_wait(fullA_bar(sa), pa);
           tc_fence_after();
@@ -622,14 +604,9 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
               tc_fence_after();
             }
             for (int kw = 0; kw < 3; ++kw) {
-              uint32_t b_base;
-              if (BRES) {
-                b_base = smem_base + (kh * 3 + kw) * 2 * Cfg::B_PLANE_BYTES;
-              } else {
-                mbar_wait(fullB_bar(sb), pb);
-                tc_fence_after();
-                b_base = smem_base + Cfg::SA_STAGES * Cfg::SA_BYTES + sb * Cfg::SB_BYTES;
-              }
+              mbar_wait(fullB_bar(sb), pb);
+              tc_fence_after();
+              const uint32_t b_base = smem_base + Cfg::SA_STAGES * Cfg::SA_BYTES + sb * Cfg::SB_BYTES;
               // tap kw = the strip shifted by kw pixel rows.  Measured on B200: the tensor core derives the 128B-swizzle
               // XOR from the absolute shared-memory address bits (like TMA does when it writes the strip), so a start
               // address that is 128-byte but not 1024-byte aligned just works with base-offset 0; putting the row phase
@@ -659,10 +636,8 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
                   umma_f16(d_tmem, a_hi + ko, b_hi + ko, idesc, 1u);
                 }
               }
-              if (!BRES) {
-                if (PAIR) umma2_commit_mc(emptyB_bar(sb)); else umma_commit(emptyB_bar(sb));
-                if (++sb == Cfg::SB_STAGES) { sb = 0; pb ^= 1u; }
-              }
+              if (PAIR) umma2_commit_mc(emptyB_bar(sb)); else umma_commit(emptyB_bar(sb));
+              if (++sb == Cfg::SB_STAGES) { sb = 0; pb ^= 1u; }
             }
             if (kh == 2 && cc == p.cchunks - 1) {                                // output row r complete
               if (PAIR) umma2_commit_mc(tfull_bar(slot)); else umma_commit(tfull_bar(slot));
@@ -688,31 +663,15 @@ tc_igemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_const
       bx.x = p.stride * tc.tx * p.Wt + dx; bx.y = p.stride * tc.ty * p.Ht + dy; bx.b = tc.b;
       return bx;
     };
-    // L2 prefetch cursor PF_KB k-blocks ahead of the loads (activations only: the weights are L2 residents anyway).
-    // Measured OFF (0): a prefetch box costs the TMA unit as much as a load, and with 2-4 joint stages of 48-96 KB these
-    // tiles are not load-latency bound - the sub-pixel up convs lost 20-40 % with PF_KB = 4 (profiles/microbench_r2_*).
-#ifndef FEMASR_PF_KB
-#define FEMASR_PF_KB 0
-#endif
-    constexpr int PF_KB = FEMASR_PF_KB;
-    int pf_it = 0, pf_kb = p.kb_begin;
-    auto prefetch_next = [&]() {
-      const int w = work_of(pf_it);
-      if (w < 0) return;
-      const TileCoord t = decode(w);
-      const ABox bx = a_box(t, pf_kb);
-      tma_prefetch_4d(&map_a_hi, bx.c0, bx.x, bx.y, bx.b);
-      tma_prefetch_4d(&map_a_lo, bx.c0, bx.x, bx.y, bx.b);
-      if (++pf_kb == p.kb_end) { pf_kb = p.kb_begin; ++pf_it; }
-    };
-    for (int i = 0; i < PF_KB; ++i) prefetch_next();
+    // No L2 prefetch ahead of these loads (unlike the strip producer): a prefetch box costs the TMA unit as much as a
+    // load, and with 2-4 joint stages of 48-96 KB these tiles are not load-latency bound - the sub-pixel up convs lost
+    // 20-40 % with a prefetch 4 k-blocks ahead (profiles/microbench_r2_*).
     for (int it = 0, work; (work = work_of(it)) >= 0; ++it) {
       const TileCoord tc = decode(work);
       const int n0 = tc.ph * p.Cout + tc.nt * BN + (PAIR ? (int)rank * (BN / 2) : 0);
       for (int kb = p.kb_begin; kb < p.kb_end; ++kb) {
         const ABox bx = a_box(tc, kb);
         const int tap = bx.tap, c0 = bx.c0;
-        if (PF_KB > 0) prefetch_next();
         mbar_wait(empty_bar(stage), phase ^ 1u);
         const uint32_t sa = smem_base + stage * Cfg::STAGE_BYTES;
         if (PAIR) {
@@ -1199,8 +1158,6 @@ template <int MODE>
 __global__ void __launch_bounds__(256) tc_prepare_flat_kernel(const float4* __restrict__ x, uint2* __restrict__ hi,
                                                               uint2* __restrict__ lo, const float* __restrict__ sc,
                                                               const float* __restrict__ sh, int C, int per_image4) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int b = blockIdx.y;
   const long base = (long)b * per_image4;
   const int i0 = blockIdx.x * (256 * PREP_U) + threadIdx.x;
@@ -1214,7 +1171,9 @@ __global__ void __launch_bounds__(256) tc_prepare_flat_kernel(const float4* __re
 #pragma unroll
   for (int u = 0; u < PREP_U; ++u) {
     const int i = i0 + u * 256;
-    if (i >= per_image4) break;
+    // `continue`, not `break` (same result: i grows with u): with `break` the optimiser sinks each load above next to its
+    // use, and the fast-SiLU variant kept one request in flight instead of PREP_U (27 instead of 40 registers)
+    if (i >= per_image4) continue;
     float w[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
     if (MODE == FEMASR_PRO_GN_SILU || MODE == FEMASR_PRO_GN_SILU_FAST) {
       const int c = (i % c4) * 4;
@@ -1319,8 +1278,6 @@ __global__ void __launch_bounds__(256) tc_prepare_flat_f8_kernel(const float4* _
 __global__ void __launch_bounds__(256) tc_prepare_ln_kernel(const float* __restrict__ x, __half* __restrict__ hi,
                                                             __half* __restrict__ lo, const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, long M, float eps) {
-  pdl_launch_dependents();
-  pdl_wait();
   // two rows per warp, all four 512-byte requests of the warp in flight before the first reduction (the one-row version
   // ran at 5.2 TB/s against 6.5-6.9 of the flat staging kernels)
   constexpr int LN_ROWS = 2;
@@ -1480,33 +1437,16 @@ static int make_map(CUtensorMap* m, const void* ptr, int rank, const cuuint64_t*
   return FEMASR_OK;
 }
 
-// Launch with the programmatic-stream-serialisation attribute when FEMASR_PDL=1.  Only kernels that execute
-// griddepcontrol.wait before their first dependent global access are launched this way.  OFF by default: measured on
-// the whole step (same box, CUDA-graph replay, profiles/bench_r2_pdl_ab.json) 78.5 ms without, 81.3 ms with it - the
-// persistent 227 KB CTAs cannot become resident before the predecessor's retire anyway, so only the (already short)
-// launch gap is exposed to overlap, and the early-launched grids cost more than that saves.
-static bool pdl_enabled() {
-  static const int env = [] { const char* e = getenv("FEMASR_PDL"); return e ? atoi(e) : 0; }();
-  return env != 0;
-}
+// Launch in clusters of cluster_x CTAs along x (2: the CTA pairs of the cta_group::2 kernels; 1: a plain launch).
 template <class... KArgs, class... Args>
-static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster_x,
-                              Args&&... args) {
+static cudaError_t launch_clustered(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                   int cluster_x, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int n = 0;
-  if (cluster_x > 1) {
-    attr[n].id = cudaLaunchAttributeClusterDimension;
-    attr[n].val.clusterDim.x = cluster_x; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = 1;
-    ++n;
-  }
-  if (pdl_enabled()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  cfg.attrs = attr; cfg.numAttrs = n;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = cluster_x; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+  cfg.attrs = &attr; cfg.numAttrs = cluster_x > 1 ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -1524,7 +1464,7 @@ static int launch_tc_v(const CUtensorMap& ah, const CUtensorMap& al, const CUten
   }
   if constexpr (!PAIR) {
     const int grid = p.num_tiles < sm_count() ? p.num_tiles : sm_count();
-    FEMASR_CUDA(launch_pdl(tc_igemm_kernel<BN, false, STRIP, BRES, RES>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 1,
+    FEMASR_CUDA(launch_clustered(tc_igemm_kernel<BN, false, STRIP, BRES, RES>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 1,
                            ah, al, bh, bl, om.y, om.oh, om.ol, p));
     return launch_status("tc_igemm_kernel");
   } else {
@@ -1532,7 +1472,7 @@ static int launch_tc_v(const CUtensorMap& ah, const CUtensorMap& al, const CUten
     const int phases = p.up ? 4 : 1;
     const int work = phases * ((num_m / phases + 1) / 2) * p.n_tiles;
     const int pairs = work < sm_count() / 2 ? work : sm_count() / 2;
-    FEMASR_CUDA(launch_pdl(tc_igemm_kernel<BN, true, STRIP, false, RES>, dim3(2 * pairs), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 2,
+    FEMASR_CUDA(launch_clustered(tc_igemm_kernel<BN, true, STRIP, false, RES>, dim3(2 * pairs), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 2,
                            ah, al, bh, bl, om.y, om.oh, om.ol, p));
     return launch_status("tc_igemm_kernel(pair)");
   }
@@ -1556,7 +1496,7 @@ static int launch_vq(const CUtensorMap& ah, const CUtensorMap& al, const CUtenso
   }
   const int num_m = p.num_tiles / p.n_tiles;
   const int grid = num_m < sm_count() ? num_m : sm_count();
-  FEMASR_CUDA(launch_pdl(tc_igemm_kernel<BN, false, false, false, false, true>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 1,
+  FEMASR_CUDA(launch_clustered(tc_igemm_kernel<BN, false, false, false, false, true>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 1,
                          ah, al, bh, bl, ah, ah, ah, p));
   return launch_status("tc_igemm_kernel(vq)");
 }
@@ -1582,40 +1522,32 @@ static TilePlan plan_tiles(const femasr_tc_args* a, int H, int W) {
   const int stride = a->stride == 2 ? 2 : 1;
   const int taps = a->upsample ? 4 : a->ksize * a->ksize;
   t.BN = a->Cout % 256 == 0 ? 256 : (a->Cout % 128 == 0 ? 128 : 64);
-  // study knob: FEMASR_TC_BN caps the tile width (e.g. 128-wide tiles for the 256-wide layers)
-  static const int bn_env = [] { const char* e = getenv("FEMASR_TC_BN"); return e ? atoi(e) : 0; }();
-  if ((bn_env == 128 || bn_env == 64) && bn_env < t.BN && a->Cout % bn_env == 0) t.BN = bn_env;
-  // CTA pairs (tcgen05 cta_group::2): a->pair 1 = on, 0 = off, -1 = automatic (FEMASR_TC_PAIR=0/1 overrides).
+  // CTA pairs (tcgen05 cta_group::2): a->pair 1 = on, 0 = off, -1 = automatic.
   // Measured (profiles/microbench_*): pairing pays when the weight tile is wide and the K loop long enough to
   // amortise the pair's coupling - BN = 256 and K >= 1024 (+10..22 %); narrow / short-K layers are faster unpaired.
-  static const int pair_env = [] { const char* e = getenv("FEMASR_TC_PAIR"); return e ? atoi(e) : -1; }();
-  const int pair_req = a->pair >= 0 ? a->pair : pair_env;
   // Round-2 sweep with the cheap (elect.sync) MMA issue (profiles/sweep_bn_pair_r2.txt): the plain fp32-output linears with
   // three or more column tiles (qkv) also gain 5 % paired; fc1 (GELU + split epilogue, issue-bound) and proj do not.
   const bool wide_plain_linear = a->ksize == 1 && a->act == FEMASR_ACT_NONE && a->y && a->Cout >= 768;
-  t.pair = pair_req >= 0 ? pair_req != 0 : (t.BN == 256 && ((long)taps * a->Cin >= 1024 || wide_plain_linear));
+  t.pair = a->pair >= 0 ? a->pair != 0 : (t.BN == 256 && ((long)taps * a->Cin >= 1024 || wide_plain_linear));
   // K-sliced layers (in front of the VQ): 128-wide tiles - the accumulator drain of a slice is half as long, twice as
   // many tiles overlap it (fc2 0.210 -> 0.197 ms),
   // and with 128-wide tiles the three-buffer protocol applies (the MMA no longer waits for the fold): fc2 0.213 -> 0.181,
   // 256 -> 256 @64² sliced conv 0.367 -> 0.319 ms paired (profiles/sweep_bn_pair_r2.txt)
-  if (bn_env == 0 && a->slice_kb > 0 && t.BN == 256 && pair_req < 0) {
+  if (a->slice_kb > 0 && t.BN == 256 && a->pair < 0) {
     t.BN = 128;
     t.pair = a->ksize == 3 && (long)taps * a->Cin >= 1024;
   }
-  // strip mode (one activation strip shared by the three horizontal taps): a->strip 1/0/-1 like pair
-  static const int strip_env = [] { const char* e = getenv("FEMASR_TC_STRIP"); return e ? atoi(e) : -1; }();
-  const int strip_req = a->strip >= 0 ? a->strip : strip_env;
+  // strip mode (one activation strip shared by the three horizontal taps) wherever the layer allows it; a->strip 0 turns
+  // it off, like a->pair
   const bool strip_ok = a->ksize == 3 && stride == 1 && !a->upsample && t.BN <= 128 && W >= 128 && a->kb_begin == 0 &&
                         a->kb_count == 0 && a->slice_kb == 0;
-  t.strip = strip_ok && (strip_req >= 0 ? strip_req != 0 : true);
+  t.strip = strip_ok && a->strip != 0;
   if (t.strip) {
     // strips over a CTA pair (two neighbouring row tiles share every weight tile, each CTA stages half of it): 128-wide
-    // tiles with streamed weights only.  Default on (FEMASR_TC_STRIP_PAIR=0 / a->pair = 0: single-CTA strips): the
-    // 128 -> 128 @256² convs re-stream the whole 590 KB weight matrix per row tile and are L2-bound in F8 mode;
-    // same-box: 1.156 -> 1.056 ms (F8), 1.490 -> 1.412 ms (three fp16 products), bit-identical results
-    static const int sp_env = [] { const char* e = getenv("FEMASR_TC_STRIP_PAIR"); return e ? atoi(e) : -1; }();
-    const bool bres_like = a->Cin == 64 && a->Cout == 64;
-    t.pair = t.BN == 128 && !bres_like && (pair_req >= 0 ? pair_req != 0 : (sp_env >= 0 ? sp_env != 0 : true));
+    // tiles with streamed weights only, unless a->pair = 0 asks for single-CTA strips.  The 128 -> 128 @256² convs
+    // re-stream the whole 590 KB weight matrix per row tile and are L2-bound in F8 mode; same-box: 1.156 -> 1.056 ms
+    // (F8), 1.490 -> 1.412 ms (three fp16 products), bit-identical results
+    t.pair = t.BN == 128 && a->pair != 0;
     t.Wt = 128; t.Ht = 1;
   } else {
     tc_tile_shape(H, W, &t.Wt, &t.Ht);   // the widest power-of-two Wt <= 128 that wastes the fewest padded pixels
@@ -1722,23 +1654,24 @@ extern "C" int femasr_tc_prepare(const float* x, void* a_hi, void* a_lo, int mod
   if (mode == FEMASR_PRO_LN) {
     FEMASR_CHECK_ARG(C == 256 && gamma && beta && !upsample, "tc_prepare: LN mode needs C=256, gamma/beta, no upsample");
     const long M = (long)B * H * W;
-    FEMASR_CUDA(launch_pdl(tc_prepare_ln_kernel, dim3((unsigned)cdiv(M, 16)), dim3(256), 0, st, 1, x, hi, lo, gamma, beta, M, eps));
+    tc_prepare_ln_kernel<<<(unsigned)cdiv(M, 16), 256, 0, st>>>(x, hi, lo, gamma, beta, M, eps);
     return launch_status("tc_prepare_ln_kernel");
   }
-  static const int flat_env = [] { const char* e = getenv("FEMASR_PREP_FLAT"); return e ? atoi(e) : 1; }();
-  if (!upsample && flat_env && (long)H * W * (C / 4) < (1l << 30) && B <= 65535 &&
+  if (!upsample && (long)H * W * (C / 4) < (1l << 30) && B <= 65535 &&
       (mode == FEMASR_PRO_GN_SILU || mode == FEMASR_PRO_GN_SILU_FAST || mode == FEMASR_PRO_NONE)) {
     const int per4 = H * W * (C / 4);
     const dim3 grid((unsigned)cdiv(per4, 256 * PREP_U), (unsigned)B);
     const float4* x4 = reinterpret_cast<const float4*>(x);
+    uint2* hi2 = reinterpret_cast<uint2*>(hi);
+    uint2* lo2 = reinterpret_cast<uint2*>(lo);
     if (mode == FEMASR_PRO_GN_SILU) {
       FEMASR_CHECK_ARG(pro_a && pro_b, "tc_prepare: GN mode needs the scale/shift tables");
-      FEMASR_CUDA(launch_pdl(tc_prepare_flat_kernel<FEMASR_PRO_GN_SILU>, grid, dim3(256), 0, st, 1, x4, reinterpret_cast<uint2*>(hi), reinterpret_cast<uint2*>(lo), pro_a, pro_b, C, per4));
+      tc_prepare_flat_kernel<FEMASR_PRO_GN_SILU><<<grid, 256, 0, st>>>(x4, hi2, lo2, pro_a, pro_b, C, per4);
     } else if (mode == FEMASR_PRO_GN_SILU_FAST) {
       FEMASR_CHECK_ARG(pro_a && pro_b, "tc_prepare: GN mode needs the scale/shift tables");
-      FEMASR_CUDA(launch_pdl(tc_prepare_flat_kernel<FEMASR_PRO_GN_SILU_FAST>, grid, dim3(256), 0, st, 1, x4, reinterpret_cast<uint2*>(hi), reinterpret_cast<uint2*>(lo), pro_a, pro_b, C, per4));
+      tc_prepare_flat_kernel<FEMASR_PRO_GN_SILU_FAST><<<grid, 256, 0, st>>>(x4, hi2, lo2, pro_a, pro_b, C, per4);
     } else {
-      FEMASR_CUDA(launch_pdl(tc_prepare_flat_kernel<FEMASR_PRO_NONE>, grid, dim3(256), 0, st, 1, x4, reinterpret_cast<uint2*>(hi), reinterpret_cast<uint2*>(lo), (const float*)nullptr, (const float*)nullptr, C, per4));
+      tc_prepare_flat_kernel<FEMASR_PRO_NONE><<<grid, 256, 0, st>>>(x4, hi2, lo2, nullptr, nullptr, C, per4);
     }
     return launch_status("tc_prepare_flat_kernel");
   }
@@ -1843,9 +1776,8 @@ extern "C" int femasr_tc_igemm(const femasr_tc_args* a, void* stream) {
   const bool pair = plan.pair, strip = plan.strip;
   FEMASR_CHECK_ARG(!(a->strip == 1 && !strip), "tc_igemm: strip mode needs a plain 3x3 stride-1 conv, Cout tile <= 128, W >= 128, no K slicing");
   p.gn_rows = phases * p.tiles_x * p.tiles_y * 4;           // one partial row per (128-pixel tile, lane quarter)
-  // 64 -> 64 channels: weights resident in shared memory, work items of 4 image rows (FEMASR_TC_BRES=0: streamed weights)
-  static const int bres_env = [] { const char* e = getenv("FEMASR_TC_BRES"); return e ? atoi(e) : 1; }();
-  const bool bres = strip && bres_env && a->Cin == 64 && a->Cout == 64;
+  // 64 -> 64 channels: weights resident in shared memory, work items of 4 image rows
+  const bool bres = strip && a->Cin == 64 && a->Cout == 64;
   if (bres) p.tiles_y = (int)cdiv(H, TcCfg<64, false, true, true>::MR);
   const long ntile = (long)phases * B * p.tiles_x * p.tiles_y * p.n_tiles;
   FEMASR_CHECK_ARG(ntile < (1l << 31), "tc_igemm: too many tiles");
@@ -1878,7 +1810,6 @@ extern "C" int femasr_tc_igemm(const femasr_tc_args* a, void* stream) {
   }
   // TMA-store epilogue: the output is a plain [B, H, W, Cout] tensor (no sub-pixel phases) -> the staging tile of each
   // epilogue warp (32 accumulator rows x 16 columns) leaves as one bulk tensor store; edge tiles are clipped by the TMA
-  static const int tma_env = [] { const char* e = getenv("FEMASR_TMA_STORE"); return e ? atoi(e) : 1; }();
   OutMaps om;
   om.y = mah; om.oh = mah; om.ol = mah;
   p.tma_out = 0;
@@ -1886,8 +1817,8 @@ extern "C" int femasr_tc_igemm(const femasr_tc_args* a, void* stream) {
   p.box_w_shift = 0; while ((1 << p.box_w_shift) < p.box_w) ++p.box_w_shift;
   // Measured same-box A/B (profiles/microbench_r2_tma_store_ab.txt): linears +3..6 %, 64-wide strip convs -5..9 % (8
   // epilogue warps: the extra staging write and the read-wait of the bulk store cost more than the stores they replace),
-  // other convs neutral -> enabled for ksize 1 only; FEMASR_TMA_STORE=2 forces it everywhere, 0 disables it.
-  if (tma_env && !a->upsample && (a->ksize == 1 || tma_env == 2)) {
+  // other convs neutral -> enabled for ksize 1 only.
+  if (a->ksize == 1 && !a->upsample) {
     const cuuint64_t dims[4] = {(cuuint64_t)a->Cout, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
     const cuuint32_t box[4] = {16, (cuuint32_t)p.box_w, (cuuint32_t)(32 / p.box_w), 1};
     if (a->y) {

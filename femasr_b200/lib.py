@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("FEMASR_LIB") or os.path.join(_HERE, "libfemasr_b200.so")
 
 PRO_NONE, PRO_GN_SILU, PRO_LN, PRO_GN_SILU_FAST = 0, 1, 2, 3
-ABI_VERSION = 4          # femasr_abi_version() of the library this binding was written against (include/femasr_b200.h)
+ABI_VERSION = 5          # femasr_abi_version() of the library this binding was written against (include/femasr_b200.h)
 ACT_NONE, ACT_GELU = 0, 1
 TAP_STAGES = ("in_conv", "down", "swin", "up1", "up2", "z", "zq", "after_quant", "dec0", "dec1", "dec2")
 
@@ -110,7 +110,6 @@ SIGNATURES = {
     "femasr_gram_diff": (_I, [_V, _V, _V, _I, _I, _I, _V]),
     "femasr_codebook_gather": (_I, [_V, _V, _V, _I, _I, _I, _V]),
     "femasr_in_conv4x4": (_I, [_V, _V, _V, _V, _I, _I, _I, _I, _I, _V]),
-    "femasr_in_conv4x4_split": (_I, [_V, _V, _V, _V, _V, _I, _I, _I, _I, _I, _V]),
     "femasr_in_conv_im2col": (_I, [_V, _V, _V, _I, _I, _I, _I, _V]),
     "femasr_in_conv_pad_weight": (_I, [_V, _V, _I, _V]),
     "femasr_out_conv3x3": (_I, [_V, _V, _V, _V, _I, _I, _I, _I, _V]),

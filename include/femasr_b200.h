@@ -308,9 +308,6 @@ int femasr_codebook_gather(const int64_t* idx, const float* codebook, float* zq,
  * w packed [16*Cin][Cout]. */
 int femasr_in_conv4x4(const float* x_nchw, const float* w, const float* bias, float* y_nhwc, int B,
                       int Cin, int H, int W, int Cout, void* stream);
-/* same, but the result is written as the split fp16 operand planes of the following tensor-core conv */
-int femasr_in_conv4x4_split(const float* x_nchw, const float* w, const float* bias, void* y_hi, void* y_lo, int B,
-                            int Cin, int H, int W, int Cout, void* stream);
 /* in_conv on the tensor cores (femasr_arch.py:150): femasr_in_conv_im2col writes, per output pixel of the 4x4 p1 conv,
  * its 48 input values (k = (kh*4+kw)*3+ci, zero padded to 64) as split fp16 planes [B*(H-1)*(W-1)][64]; the conv is then
  * femasr_tc_igemm with ksize 1, Cin 64 on a weight blob packed from femasr_in_conv_pad_weight's [Cout][64] matrix. */

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """GPU-box study behind tests/test_fullsize_gpu.py: codebook-index differences against the CPU oracle at the FULL benchmark
-geometry (x4, 128x128, batch 32 = 131072 VQ rows, default tie-heavy init) for several arithmetic variants of the engine,
+geometry (x4, 128x128, batch 32 = 131072 VQ rows, default tie-heavy init) for the tensor-core path and the fp32 path,
 each classified by the ORACLE's own fp32 distances: a difference is "tie-equivalent" when the oracle's distance of our
 code is within `k` grid steps (ulp of A = sum z^2) of the oracle's best - i.e. the two codes are separated by less than
 the rounding noise of ANY fp32 evaluation order (the oracle itself moves this many rows when its thread count changes,
@@ -21,10 +21,6 @@ sys.path.insert(0, ROOT)
 
 VARIANTS = {
     "default (tcgen05, K-slice 256)": {},
-    "tcgen05, K-slice 128": {"FEMASR_TC_SLICE_KB": "2"},
-    "tcgen05, K-slice 64": {"FEMASR_TC_SLICE_KB": "1"},
-    "tcgen05, no K-slicing": {"FEMASR_TC_PRECISE": "0"},
-    "tcgen05, VQ on fp32 SIMT": {"FEMASR_VQ_FUSED": "0"},
     "fp32 FFMA path (gemm_path=0)": {"FEMASR_GEMM_PATH": "0"},
 }
 

@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol(built_lib):
     for n in names:
         assert hasattr(dll, n), f"{n} declared in the header but not exported"
     assert sorted(lib.SIGNATURES) == names, "femasr_b200/lib.py SIGNATURES out of sync with the header"
-    assert lib.load().femasr_abi_version() == lib.ABI_VERSION == 4
+    assert lib.load().femasr_abi_version() == lib.ABI_VERSION == 5
 
 
 def test_argument_validation_without_gpu(built_lib):

@@ -1,4 +1,4 @@
-"""CPU model of the MMA schedule of the resident-weight 64 -> 64 strip kernel (femasr_b200/csrc/tc_gemm.cu, BRES_MERGE):
+"""CPU model of the MMA schedule of the resident-weight 64 -> 64 strip kernel (femasr_b200/csrc/tc_gemm.cu, the merged tap-row schedule):
 the merged form (one MMA of N = 64 x rows per input strip, kw, k-step and product) must hand every accumulator exactly the
 contributions of the unmerged form, in the same order, and read them from the right weight plane of the merged layout.
 Mirrors the index arithmetic of the kernel; the GPU proof is scripts/ab_digest.py (bit-identical outputs)."""

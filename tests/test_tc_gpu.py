@@ -193,20 +193,6 @@ def test_tc_strip_mode(cuda, B, H, W, Cin, Cout):
                            G.tc_igemm(h8, x8, b8, bg, Cout, 3, res1=res, strip=1, pair=1, f8=1))
 
 
-def test_in_conv_split_planes(cuda):
-    lib = L.load()
-    B, H, W, cout = 2, 18, 23, 256
-    x, w, b = torch.rand(B, 3, H, W), rnd(cout, 3, 4, 4, seed=36, scale=0.15), rnd(cout, seed=37)
-    want = F.conv2d(x, w, b, padding=1)
-    hi = torch.empty(B, H - 1, W - 1, cout, dtype=torch.float16, device=cuda)
-    lo = torch.empty_like(hi)
-    xg, wp, bg = x.to(cuda), G.pack_weight(w.to(cuda)), b.to(cuda)
-    L.check(lib.femasr_in_conv4x4_split(xg.data_ptr(), wp.data_ptr(), bg.data_ptr(), hi.data_ptr(), lo.data_ptr(),
-                                        B, 3, H, W, cout, G.S()))
-    got = (hi.float() + lo.float()).permute(0, 3, 1, 2).cpu()
-    assert (got - want).abs().max().item() <= 5e-6
-
-
 def test_tc_split_output(cuda):
     M, K, N = 500, 256, 1024
     x, w, b = rnd(M, K, seed=24), rnd(N, K, seed=25, scale=0.05), rnd(N, seed=26)
